@@ -3,14 +3,16 @@
 pool-sharded over the N GPUs), plus wall-clock to 1e-6 relative gap, the HBM roofline of the dominant kernel, and the
 CPU baseline timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaling strong|weak]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaling strong|weak] [--dump-outputs DIR]
 
 A "step" is one dual evaluation of the problem: the per-pool optimal-arbitrage kernel over this rank's pools,
 accumulating psi(nu) and the dual value, + (N > 1) the one all-reduce of the (n_tokens+1)-vector.  Default scaling is
 STRONG: the 1M pools are split over the N GPUs (BASELINE.json configs[4]); the weak-scaled figure (1M pools per GPU)
 rides along as the `weak` key at N > 1.  Steps rotate over independent pool instances resident on each GPU, enough of
-them to exceed the 126 MB L2 (>= 256 MiB), so every step streams its pools from HBM.  The K timed steps are replayed
-from CUDA graphs of min(K, 64) steps for any K.  One JSON line on stdout (rank 0).
+them to exceed the 126 MB L2 (>= 256 MiB), so every step streams its pools from HBM.  Exactly K steps are timed, replayed
+from CUDA graphs.  One JSON line on stdout (rank 0).  --dump-outputs DIR writes what the last timed step returned, psi(nu)
+as DIR/psi.npy and the dual value's arbitrage term as DIR/arb.npy (float64); the inputs are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -223,15 +225,17 @@ def workload_config(n_gpus, scaling, n_inst):
 
 # --------------------------------------------------------------------------------------------------
 def timed_steps(step, steps, warmup, barrier, clock_index, n_inst, preroll_ms=40.0):
-    """W warm-up steps, then exactly `steps` steps replayed from CUDA graphs of min(steps, 64) steps, CUDA-event timed,
-    barrier + synchronize on both sides.  The clock sampler also covers a pre-roll of the same graph (the timed region
-    itself is too short for NVML's sampling interval).  Returns (ms_total, steps_timed, clocks)."""
+    """W warm-up steps, then exactly `steps` steps replayed from CUDA graphs, CUDA-event timed, barrier + synchronize on
+    both sides: a graph of CHUNK steps replayed steps // CHUNK times, then one graph of the steps % CHUNK left.  CHUNK is
+    a multiple of 2 n_inst: every store is evaluated an even number of times per replay, so the ping-pong accumulator each
+    call clears for the next one (PoolStore.evaluate) is the one the replayed graph starts from.  The clock sampler also
+    covers a pre-roll of the CHUNK graph (the timed region itself is too short for NVML's sampling interval).
+    Returns (ms_total, steps_timed, clocks, what the last timed step returned)."""
     import torch
     for i in range(max(warmup, 3)):
         step(i)
     barrier()
-    CHUNK = min(steps, 64)
-    steps = (steps // CHUNK) * CHUNK
+    CHUNK = max(1, 64 // (2 * n_inst)) * 2 * n_inst
     side = torch.cuda.Stream()
     side.wait_stream(torch.cuda.current_stream())
     with torch.cuda.stream(side):
@@ -242,7 +246,13 @@ def timed_steps(step, steps, warmup, barrier, clock_index, n_inst, preroll_ms=40
     graph = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph):
         for i in range(CHUNK):
-            step(i)
+            last = step(i)
+    tail = None
+    if steps % CHUNK:            # steps CHUNK * (steps // CHUNK) + i use instance i mod n_inst, as in the CHUNK graph
+        tail = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(tail):
+            for i in range(steps % CHUNK):
+                last = step(i)
     graph.replay()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -259,10 +269,12 @@ def timed_steps(step, steps, warmup, barrier, clock_index, n_inst, preroll_ms=40
         e0.record()
         for _ in range(steps // CHUNK):
             graph.replay()
+        if tail is not None:
+            tail.replay()
         e1.record()
         barrier()
         torch.cuda.profiler.stop()
-    return e0.elapsed_time(e1), steps, clocks.summary()
+    return e0.elapsed_time(e1), steps, clocks.summary(), last
 
 
 def build_instances(I, cf, dev, rank, world, per, scaling, n_inst):
@@ -374,7 +386,8 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     def measure(scaling):
-        """the timed evaluation steps for one scaling mode: (ms_per_step, steps, clocks, eval-only ms_per_step, store)"""
+        """the timed evaluation steps for one scaling mode: (ms_per_step, steps, clocks, eval-only ms_per_step, store, ...,
+        the last timed step's [psi | arb] on the host)"""
         per = M_POOLS if scaling == "weak" else M_POOLS // world
         n_inst = n_instances(per)
         stores, nus = build_instances(I, cf, dev, rank, world, per, scaling, n_inst)
@@ -394,24 +407,29 @@ def run_b200(args):
                 dist.all_reduce(acc)
             return acc
 
-        ms, steps, clocks = timed_steps(step, args.steps, args.warmup, barrier, local, n_inst)
+        ms, steps, clocks, last = timed_steps(step, args.steps, args.warmup, barrier, local, n_inst)
+        last = last.cpu().numpy()
         t = torch.tensor([ms], **f64)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         eval_only = None
         if world > 1:            # the same steps without the collective: the all-reduce share of a step
-            ms0, steps0, _ = timed_steps(lambda i: stores[i % n_inst].evaluate(nus[i % n_inst], reduce=False), args.steps,
-                                         args.warmup, barrier, local, n_inst, preroll_ms=10.0)
+            ms0, steps0, _, _ = timed_steps(lambda i: stores[i % n_inst].evaluate(nus[i % n_inst], reduce=False), args.steps,
+                                            args.warmup, barrier, local, n_inst, preroll_ms=10.0)
             t0 = torch.tensor([ms0], **f64); dist.all_reduce(t0, op=dist.ReduceOp.MAX)
             eval_only = float(t0) / steps0
-        return float(t) / steps, steps, clocks, eval_only, stores[0], per, n_inst, use_peer
+        return float(t) / steps, steps, clocks, eval_only, stores[0], per, n_inst, use_peer, last
 
-    ms_per_step, steps, clocks, eval_only_ms, store0, per, n_inst, used_peer = measure(args.scaling)
+    ms_per_step, steps, clocks, eval_only_ms, store0, per, n_inst, used_peer, last = measure(args.scaling)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "psi.npy"), np.asarray(last[:N_TOKENS], np.float64))
+        np.save(os.path.join(args.dump_outputs, "arb.npy"), np.asarray(last[N_TOKENS:], np.float64))
     value = n_gpus * per / (ms_per_step * 1e-3)
     weak = None
     if world > 1 and args.scaling == "strong" and not args.no_weak:
         torch.cuda.empty_cache()
-        w_ms, w_steps, _, w_eval_only, _, w_per, w_inst, _ = measure("weak")
+        w_ms, w_steps, _, w_eval_only, _, w_per, w_inst, _, _ = measure("weak")
         weak = {"value": n_gpus * w_per / (w_ms * 1e-3), "unit": UNIT, "ms_per_step": w_ms, "pools_per_gpu": w_per,
                 "pools_total": n_gpus * w_per, "eval_only_us": 1e3 * w_eval_only if w_eval_only else None,
                 "allreduce_us": 1e3 * (w_ms - w_eval_only) if w_eval_only else None, "instances_per_gpu": w_inst}
@@ -509,8 +527,8 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=6400)
-    ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 6400; --impl reference: 10)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 20; --impl reference: 1)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--scaling", default="strong", choices=["weak", "strong"],
                     help="strong (default, BASELINE configs[4]): 1M pools split over the GPUs; weak: 1M pools per GPU")
@@ -520,15 +538,23 @@ def main():
     ap.add_argument("--no-weak", action="store_true", help="N>1: skip the secondary weak-scaled measurement")
     ap.add_argument("--collective", default="peer", choices=["peer", "nccl"],
                     help="N>1: cfmm_allreduce_ll over NVLink peer memory (default) or NCCL all_reduce")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/psi.npy and DIR/arb.npy (float64)")
     args = ap.parse_args()
+    reference = args.impl == "reference"
+    if args.steps is None:                        # each reference step is seconds of CPU work
+        args.steps = 10 if reference else 6400
+    if args.warmup is None:
+        args.warmup = 1 if reference else 20
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if reference and args.dump_outputs:
+        ap.error("--dump-outputs writes the B200 path's outputs; it does not apply to --impl reference")
     # safety net: a wedged collective (a rank that died, a peer that never pushes) must end the run, not hold the box
     watchdog = threading.Timer(float(os.environ.get("CFMM_BENCH_WATCHDOG_S", "900")), lambda: os._exit(3))
     watchdog.daemon = True
     watchdog.start()
-    if args.impl == "reference":
-        if args.steps > 20:
-            args.steps = 10         # each reference step is seconds of CPU work
-            args.warmup = min(args.warmup, 1)
+    if reference:
         run_reference(args)
     else:
         run_b200(args)

@@ -2,8 +2,8 @@
 
 CPU tier: the recogniser (expression graph -> the literals of api.solve) on models wired the way the reference scripts
 wire them (arbitrage.py:38-78, liquidation.py:38-81, two-asset.py:40-87), the write-back of `.value`s with the ORACLE
-installed as the checker back end, the error messages for models outside the routing family, and -- where the reference
-tree exists -- the three scripts themselves, unmodified, through `run_script`.  GPU tier: the same models with the real
+installed as the checker back end, the error messages for models outside the routing family, and a cvxpy script of the
+reference's kind (tests/routing_script.py), unmodified, through `run_script`.  GPU tier: the same models with the real
 back end against the fixture of the executed reference (tests/golden/reference_run.json)."""
 import json
 import os
@@ -19,7 +19,6 @@ from oracle import cfmm_oracle as O
 import helpers as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -276,16 +275,15 @@ def test_random_models_round_trip(with_oracle_backend):
     assert done >= 30
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "arbitrage.py")), reason="the reference tree only exists in the build container")
-def test_reference_scripts_run_unmodified_through_the_compat_module(with_oracle_backend, ref_run, capsys):
-    g = run_script.run(os.path.join(REF, "arbitrage.py"))
+def test_cvxpy_script_runs_unmodified_through_the_compat_module(with_oracle_backend, ref_run, capsys):
+    """tests/routing_script.py states the three problems of the reference's scripts with `import cvxpy as cp` and plots
+    with matplotlib; run_script serves both, and what the script reads back is the executed reference's"""
+    g = run_script.run(os.path.join(ROOT, "tests", "routing_script.py"))
     assert abs(g["prob"].value - ref_run["arbitrage"]["value"]) <= 1e-8 * ref_run["arbitrage"]["value"]
     assert g["prob"].model.local_indices == ref_run["arbitrage"]["data"]["local_indices"]
-    assert "Total output value: 21.4998" in capsys.readouterr().out
-    g = run_script.run(os.path.join(REF, "liquidation.py"))
-    assert abs(g["psi"].value[4] - ref_run["liquidation"]["value"]) <= 1e-8 * ref_run["liquidation"]["value"]
-    assert "Total liquidated value: 15.8830" in capsys.readouterr().out
-    g = run_script.run(os.path.join(REF, "two-asset.py"))
+    assert abs(g["liq_psi"].value[4] - ref_run["liquidation"]["value"]) <= 1e-8 * ref_run["liquidation"]["value"]
+    out = capsys.readouterr().out
+    assert "Total output value: 21.4998" in out and "Total liquidated value: 15.8830" in out
     np.testing.assert_allclose(g["u_t"], ref_run["two_asset"]["u_t"], rtol=1e-7, atol=1e-7)
     for k in range(5):                                                      # fixture: [t][pool][slot]; two-asset.py:93-94
         np.testing.assert_allclose(g["all_values"][k], np.array([flows_t[k] for flows_t in ref_run["two_asset"]["flows"]]).T, atol=5e-5)

@@ -41,6 +41,7 @@ def test_c_abi_library_loads_and_exports_every_declared_symbol():
     # batch entry points: NULL / size / kind checks, work-buffer arithmetic (12 n + 2 n^2 + n(n+1) + 2 nnz doubles per lane)
     assert lib.cfmm_batch_solve(None, None, None, None, None) == -1
     cp = _lib.CsrPools(3, 5, 13, None, None, None, None, None, None, None)
+    assert lib.cfmm_set_batch_lanes(1) == 0         # the lane count is process-wide: a batch solve run earlier sets it
     assert lib.cfmm_batch_solve_work_bytes(ctypes.byref(cp), 50, 0) == 8 * (36 + 18 + 12 + 26) * 64
     assert lib.cfmm_batch_solve_work_bytes(ctypes.byref(cp), 50, 6) == 8 * (36 + 18 + 12 + 12) * 64
     assert lib.cfmm_set_batch_lanes(5) == -2 and lib.cfmm_set_batch_lanes(32) == 0

@@ -1,8 +1,8 @@
 """The oracle (and, on the GPU, the CUDA path) against outputs of the REFERENCE'S OWN SCRIPTS.
 
-tests/golden/reference_run.json is written by tests/golden/make_golden_from_reference.py, which executes
-/root/reference/{arbitrage,liquidation,two-asset}.py unmodified (runpy) with oracle/cvxpy_shim.py standing in for the
-absent cvxpy.  The fixture holds what the scripts read back after prob.solve(): prob.value, psi.value,
+tests/golden/reference_run.json was written by tests/golden/make_golden_from_reference.py, which executed the
+reference's arbitrage.py, liquidation.py and two-asset.py unmodified (runpy) with oracle/cvxpy_shim.py standing in for
+the absent cvxpy.  The fixture holds what the scripts read back after prob.solve(): prob.value, psi.value,
 deltas[i].value, lambdas[i].value (arbitrage.py:84, liquidation.py:87) and, per swept amount t, obj.value and
 lambdas[k].value - deltas[k].value (two-asset.py:93-100)."""
 import json
@@ -17,7 +17,6 @@ from oracle import cvxpy_shim as cp
 import helpers as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -75,17 +74,17 @@ def test_reference_values_agree_with_the_zero_gap_certified_ones(ref_run, golden
         assert abs(ref_run["two_asset"]["u_t"][j] - golden["two_asset"][j]["value"]) <= 1e-7 * max(1.0, golden["two_asset"][j]["value"])
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF, "arbitrage.py")), reason="the reference tree only exists in the build container")
-def test_fixture_is_what_the_reference_scripts_produce_today(ref_run):
-    """re-executes /root/reference/arbitrage.py and liquidation.py and compares with the committed fixture"""
+def test_fixture_is_what_the_shim_computes_for_the_reference_problems(ref_run):
+    """tests/routing_script.py (the three problems of the reference's scripts, stated with cvxpy's API) executed the way
+    the fixture's generator executed the reference's scripts, with the shim standing in for cvxpy"""
     import importlib.util
     spec = importlib.util.spec_from_file_location("mk", os.path.join(ROOT, "tests", "golden", "make_golden_from_reference.py"))
     mk = importlib.util.module_from_spec(spec); spec.loader.exec_module(mk)
-    g = mk.run_reference_script(os.path.join(REF, "arbitrage.py"))
+    g = mk.run_reference_script(os.path.join(ROOT, "tests", "routing_script.py"))
     assert abs(g["prob"].value - ref_run["arbitrage"]["value"]) <= 1e-10
     assert "Total output value" in g["__stdout__"]
-    g = mk.run_reference_script(os.path.join(REF, "liquidation.py"))
-    assert abs(g["psi"].value[4] - ref_run["liquidation"]["value"]) <= 1e-10
+    assert abs(g["liq_psi"].value[4] - ref_run["liquidation"]["value"]) <= 1e-10
+    np.testing.assert_allclose(g["u_t"], ref_run["two_asset"]["u_t"], rtol=0, atol=1e-10)
 
 
 def test_shim_models_what_cvxpy_would():
